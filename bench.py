@@ -18,6 +18,9 @@ The same JSON line also carries
         thread count / API / placement (scripts/cpu_ref.py), N=1 only.
 `--impl reference` prints the reference arm: the same sweep, best configuration as `value`.
 `--workload NAME` restricts the run to one of the parts (faster iteration).
+`--dump-outputs DIR` writes what the timed calls returned in their last step (compressed bytes, decoded
+bytes, sizes) as DIR/<workload>.<name>.npy in float32 -- a fixed, seeded sample of each large buffer -- so that
+two builds can be compared output for output on identical inputs.
 
 Prints ONE JSON line on rank 0.
 """
@@ -50,6 +53,7 @@ SHARDED = {
 }
 CFG5 = "lz4-shuffle-cl5-8GiB-sharded"
 METRIC = "compress+decompress GB/s"
+DUMP_SAMPLES = 1 << 20        # elements kept per dumped buffer: 4 MiB of float32 each, well under 64 MB per run
 NVLINK_GBS = 770.0            # measured peer copy per direction per GPU (B200_PROFILING.md)
 
 
@@ -157,6 +161,26 @@ class near_gpu:
     def __exit__(self, *a):
         if self.saved:
             os.sched_setaffinity(0, self.saved)
+
+
+def dump_outputs(dump_dir, workload, arrays):
+    """arrays: name -> uint8 tensor or int.  Buffers longer than DUMP_SAMPLES are sampled at sorted positions drawn
+    from a fixed seed (the same positions for the same length), so that equal outputs give equal files.  Bytes are
+    written as float32; sizes as float64, which holds them exactly (float32 would round sizes above 2^24)."""
+    if not dump_dir or int(os.environ.get("RANK", "0")) != 0:
+        return
+    import numpy as np
+    import torch
+    os.makedirs(dump_dir, exist_ok=True)
+    for name, t in arrays.items():
+        path = os.path.join(dump_dir, f"{workload}.{name}.npy")
+        if not torch.is_tensor(t):
+            np.save(path, np.array([t], np.float64))
+            continue
+        if t.numel() > DUMP_SAMPLES:
+            idx = np.sort(np.random.default_rng(0).integers(0, t.numel(), DUMP_SAMPLES))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(path, t.reshape(-1).cpu().numpy().astype(np.float32))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -273,7 +297,7 @@ def timed_steps(e, comp_args, dec_args, steps):
     return ms, tc, td, cb, nb
 
 
-def bench_chunk(e, np, workload, steps, warmup, concurrent=False, env=None):
+def bench_chunk(e, np, workload, steps, warmup, concurrent=False, env=None, dump_dir=None, dump_name=None):
     """One 256 MiB chunk per rank: device-resident value, host-pinned e2e, per-kernel times, clocks."""
     torch, pkg, dev, world = e.torch, e.pkg, e.dev, e.world
     comp_name, shuf, ts, clevel, nbytes = WORKLOADS[workload]
@@ -306,6 +330,7 @@ def bench_chunk(e, np, workload, steps, warmup, concurrent=False, env=None):
         launches = pkg.launch_count() - launches0
         prof = pkg.prof_get(); pkg.set_profiling(False)
         assert cb > 0 and nb == nbytes
+        dump_outputs(dump_dir, dump_name or workload, {"compressed": d_chunk[:cb], "decompressed": d_out, "cbytes": cb})
         # timed region 2: end to end from/to pinned host memory through the C ABI
         ms_h, tc_h, td_h, cb_h, nb_h = timed_steps(e, host_args[0], host_args[1], steps)
         clocks = sampler.stop()                  # sampled over both timed regions
@@ -406,7 +431,7 @@ def measure_traffic(workload):
         return None
 
 
-def bench_sharded(e, np, name, steps, warmup):
+def bench_sharded(e, np, name, steps, warmup, dump_dir=None):
     """8 GiB as 32 chunks of 256 MiB, 32/N per GPU.  Leg 1: every rank's run is resident on its GPU and is
     compressed as one frame (blosc_b200_frame_*: 4 chunks in flight per GPU), no collective.  Leg 2 (N>1): rank 0's
     GPU holds the whole buffer, scatters it chunk by chunk over NCCL while the ranks compress, gathers the frames,
@@ -445,7 +470,7 @@ def bench_sharded(e, np, name, steps, warmup):
         return ms, tc, td, fb
 
     sweep_out, head, clocks, prof, launches = {}, None, None, None, 0
-    nst = max(2, min(steps, 5))
+    nst = steps
     for ts in sweep:
         timed(ts, 1)
         assert torch.equal(d_out, d_src), f"round trip mismatch at typesize {ts}"
@@ -460,6 +485,7 @@ def bench_sharded(e, np, name, steps, warmup):
         cb_chunk = (fb - 32 - 8 * k) // k
         sweep_out[str(ts)] = {"value": 2 * total / (ms / nst / 1e3) / 1e9, "compress_gbs": total / (tc / nst) / 1e9,
                               "decompress_gbs": total / (td / nst) / 1e9, "ratio": chunk / cb_chunk, "cbytes_per_chunk": cb_chunk}
+    dump_outputs(dump_dir, name, {f"frame_ts{sweep[-1]}": d_frame[:fb], f"decompressed_ts{sweep[-1]}": d_out, "frame_bytes": fb})
     del d_frame, d_out
 
     sg = None
@@ -534,7 +560,10 @@ def main():
     ap.add_argument("--workload", default="all", choices=["all"] + sorted(WORKLOADS) + sorted(SHARDED))
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-traffic", action="store_true", help="skip the ncu DRAM-traffic subprocess")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     import numpy as np
 
     rank = int(os.environ.get("RANK", "0"))
@@ -548,12 +577,14 @@ def main():
     e = setup(world, local_rank)
     want = lambda w: args.workload in ("all", w)
     head_wl = CFG3 if args.workload == CFG3 else CFG2
-    head = bench_chunk(e, np, head_wl, args.steps, args.warmup, concurrent=True) if (want(CFG2) or want(CFG3)) else None
-    cfg3 = bench_chunk(e, np, CFG3, args.steps, args.warmup) if (args.workload == "all" and world == 1) else None
+    dump = args.dump_outputs
+    head = bench_chunk(e, np, head_wl, args.steps, args.warmup, concurrent=True, dump_dir=dump) if (want(CFG2) or want(CFG3)) else None
+    cfg3 = bench_chunk(e, np, CFG3, args.steps, args.warmup, dump_dir=dump) if (args.workload == "all" and world == 1) else None
     fast = None
     if args.workload == "all" and getattr(e.pkg, "HAS_FAST_PARSE", False):
-        fast = bench_chunk(e, np, CFG2, args.steps, args.warmup, env={"BLOSC_B200_PARSE": "fast"})
-    cfg5 = bench_sharded(e, np, CFG5, args.steps, args.warmup) if want(CFG5) else None
+        fast = bench_chunk(e, np, CFG2, args.steps, args.warmup, env={"BLOSC_B200_PARSE": "fast"}, dump_dir=dump,
+                           dump_name=CFG2 + "-fast-parse")
+    cfg5 = bench_sharded(e, np, CFG5, args.steps, args.warmup, dump_dir=dump) if want(CFG5) else None
     if rank != 0:
         if world > 1:
             e.dist.destroy_process_group()

@@ -36,13 +36,11 @@ def orc():
 
 @pytest.fixture(scope="session")
 def ref():
-    """The unmodified reference compiled from /root/reference (oracle/_ref), if available."""
+    """The unmodified reference (oracle/_ref, built only where its sources are at hand), or None.  Tests
+    that take it run against the stored reference results in tests/golden/ and use it on top when present."""
     path = os.path.join(ROOT, "oracle", "_ref", "libblosc_ref.so")
     if not os.path.exists(path):
-        if os.path.isdir("/root/reference/blosc"):
-            _make(os.path.join(ROOT, "oracle"), "ref")
-        else:
-            pytest.skip("oracle/_ref not built and /root/reference absent")
+        return None
     lib = C.CDLL(path)
     for f in ("blosc_compress_ctx", "blosc_decompress_ctx", "blosc_getitem", "LZ4_compress_fast", "LZ4_decompress_safe",
               "blosclz_compress", "blosclz_decompress"):

@@ -1,9 +1,84 @@
-"""Deterministic test inputs (seeded) and thin ctypes helpers shared by the tests."""
+"""Deterministic test inputs (seeded), thin ctypes helpers shared by the tests, and the stored
+results of the unmodified reference (tests/golden/reference*, written by
+scripts/record_reference_golden.py from a reference build in oracle/_ref)."""
 import ctypes as C
+import functools
+import hashlib
+import json
+import os
 
 import numpy as np
 
 vp, sz, ci = C.c_void_p, C.c_size_t, C.c_int
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+
+@functools.lru_cache(None)
+def golden():
+    """The reference's results: small values and per-group digests (reference.json)."""
+    with open(os.path.join(GOLDEN, "reference.json")) as f:
+        return json.load(f)
+
+
+@functools.lru_cache(None)
+def golden_arrays(name):
+    """Frames and chunks the reference wrote (reference_<name>.npz)."""
+    with np.load(os.path.join(GOLDEN, f"reference_{name}.npz")) as z:
+        return {k: z[k] for k in z.files}
+
+
+class Transcript:
+    """What one library returned over a series of cases, kept as one digest per group of cases.
+    The reference's transcript is stored; the oracle's or the emulator's must equal it group by group."""
+
+    def __init__(self):
+        self.hashes, self.h = {}, None
+
+    def group(self, *key):
+        self.h = self.hashes["/".join(map(str, key))] = hashlib.blake2b(digest_size=8)
+
+    def add(self, *vals):
+        for v in vals:
+            self.h.update(v.tobytes() if isinstance(v, np.ndarray) else int(v).to_bytes(8, "little", signed=True))
+
+    def digests(self):
+        return {k: h.hexdigest() for k, h in self.hashes.items()}
+
+
+def check_transcript(key, t):
+    want, got = golden()["transcripts"][key], t.digests()
+    assert sorted(got) == sorted(want), (key, "cases differ from the recorded ones")
+    bad = [k for k in want if got[k] != want[k]]
+    assert not bad, f"{key}: differs from the reference in groups {bad[:8]}"
+
+
+class Api:
+    """The entry points the transcripts call, bound to the reference's names or to the oracle's."""
+
+    def __init__(self, lib, reference):
+        self.lib, self.reference = lib, reference
+        p = "" if reference else "orc_"
+        self.lz4_compress = getattr(lib, "LZ4_compress_fast" if reference else "orc_lz4_compress_fast")
+        self.lz4_decompress = getattr(lib, "LZ4_decompress_safe" if reference else "orc_lz4_decompress_safe")
+        self.blosclz_compress = getattr(lib, p + "blosclz_compress")
+        self.blosclz_decompress = getattr(lib, p + "blosclz_decompress")
+        self.getitem = getattr(lib, "blosc_getitem" if reference else "orc_getitem")
+        self.ctx = ("blosc_" if reference else "orc_") + "compress_ctx", ("blosc_" if reference else "orc_") + "decompress_ctx"
+
+    def compress(self, *args, **kw):
+        return compress(self.lib, self.ctx[0], *args, **kw)
+
+    def decompress(self, *args, **kw):
+        return decompress(self.lib, self.ctx[1], *args, **kw)
+
+    def filter(self, op, ts, n, src, dst):
+        """op: shuffle, unshuffle, bitshuffle or bitunshuffle"""
+        if not self.reference:
+            return getattr(self.lib, "orc_" + op)(sz(ts), sz(n), ptr(src), ptr(dst))
+        args = [sz(ts), sz(n), ptr(src), ptr(dst)]
+        if op.startswith("bit"):
+            args.append(ptr(np.zeros(n + 64, np.uint8)))
+        return getattr(self.lib, "blosc_internal_" + op)(*args)
 
 
 def ptr(a):

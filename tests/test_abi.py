@@ -5,6 +5,8 @@ import ctypes as C
 import os
 import re
 
+from datagen import golden
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -26,27 +28,22 @@ def _dynamic_symbols(path):
 
 def test_reference_public_symbols_present(pkg):
     """Every public blosc_* symbol of the reference is exported here.  The list SURVEY.md section 8b recorded is checked
-    against the reference's own header (BLOSC_EXPORT declarations) and against `nm -D` of the reference built from
-    /root/reference (oracle/_ref) whenever those are present."""
+    against the reference's own header (BLOSC_EXPORT declarations) and against `nm -D` of the reference build, both
+    stored in tests/golden/reference.json."""
     ref_syms = """blosc_init blosc_destroy blosc_compress blosc_compress_ctx blosc_decompress blosc_decompress_ctx
     blosc_getitem blosc_get_nthreads blosc_set_nthreads blosc_get_compressor blosc_set_compressor
     blosc_compcode_to_compname blosc_compname_to_compcode blosc_list_compressors blosc_get_version_string
     blosc_get_complib_info blosc_free_resources blosc_cbuffer_sizes blosc_cbuffer_validate blosc_cbuffer_metainfo
     blosc_cbuffer_versions blosc_cbuffer_complib blosc_get_blocksize blosc_set_blocksize blosc_set_splitmode""".split()
     assert len(ref_syms) == 25
-    hdr_path = "/root/reference/blosc/blosc.h"
-    if os.path.exists(hdr_path):
-        # the public API is what blosc.h marks BLOSC_EXPORT (everything else is hidden by -fvisibility=hidden,
-        # blosc/CMakeLists.txt:6-8): the recorded list must be exactly that
-        hdr = re.sub(r"/\*.*?\*/", "", open(hdr_path).read(), flags=re.S)
-        public = set(re.findall(r"BLOSC_EXPORT[^;(]*?\b(blosc_[a-z0-9_]+)\s*\(", hdr))
-        assert public == set(ref_syms), (sorted(public - set(ref_syms)), sorted(set(ref_syms) - public))
-    ref_path = os.path.join(ROOT, "oracle", "_ref", "libblosc_ref.so")
-    if os.path.exists(ref_path):
-        # ... and each of them is a symbol the reference build really defines (oracle/_ref is built without the
-        # visibility flag, so it exports some internals on top: those are not part of the contract)
-        defined = _dynamic_symbols(ref_path)
-        assert set(ref_syms) <= defined, sorted(set(ref_syms) - defined)
+    # the public API is what blosc.h marks BLOSC_EXPORT (everything else is hidden by -fvisibility=hidden,
+    # blosc/CMakeLists.txt:6-8): the recorded list must be exactly that
+    public = set(golden()["abi"]["header_exports"])
+    assert public == set(ref_syms), (sorted(public - set(ref_syms)), sorted(set(ref_syms) - public))
+    # ... and each of them is a symbol the reference build really defines (it is built without the visibility flag,
+    # so it exports some internals on top: those are not part of the contract)
+    defined = set(golden()["abi"]["defined"])
+    assert set(ref_syms) <= defined, sorted(set(ref_syms) - defined)
     ours = _dynamic_symbols(pkg.LIB_PATH)
     missing = [s for s in ref_syms if s not in ours]
     assert not missing, missing
@@ -81,3 +78,10 @@ def test_product_does_not_touch_the_oracle():
                     if re.search(r"#\s*include.*(oracle|simt_emu)|import.*oracle|liboracle|libblosc_ref|orc_[a-z]", line):
                         bad.append((f, line.strip()))
     assert not bad, bad
+
+
+def reference_golden(ref_path, header_path):
+    hdr = re.sub(r"/\*.*?\*/", "", open(header_path).read(), flags=re.S)
+    public = sorted(set(re.findall(r"BLOSC_EXPORT[^;(]*?\b(blosc_[a-z0-9_]+)\s*\(", hdr)))
+    defined = sorted(s for s in _dynamic_symbols(ref_path) if s.startswith("blosc_"))
+    return {"abi": {"header_exports": public, "defined": defined}}

@@ -1,13 +1,13 @@
 """Damaged / hostile input: the accept-reject verdict (and the bytes, when accepted) must be the
-reference's.  CPU: reference (oracle/_ref) vs oracle vs the product's device code in the SIMT
-emulator.  GPU: the CUDA library vs the oracle (ADVICE r1: negative header nbytes, LZ4 offset 0,
-the 9-literal rule of the batch path, frame slots)."""
+reference's.  CPU: the reference's verdicts (stored in tests/golden/reference.json) vs oracle vs the
+product's device code in the SIMT emulator.  GPU: the CUDA library vs the oracle (ADVICE r1:
+negative header nbytes, LZ4 offset 0, the 9-literal rule of the batch path, frame slots)."""
 import ctypes as C
 
 import numpy as np
 import pytest
 
-from datagen import ci, compress, gen, ptr, sz
+from datagen import Transcript, check_transcript, ci, compress, gen, golden, ptr, sz
 
 
 def _lz4_mutants(orc, rng, count):
@@ -31,32 +31,47 @@ def _lz4_mutants(orc, rng, count):
     return out
 
 
-def test_lz4_decode_verdicts_match_reference(orc, ref, emu):
+def _lz4_verdicts(orc, decode):
+    """decode(c, n, out) -> return value; one group per mutant: the verdict and, when accepted, the bytes."""
     rng = np.random.default_rng(11)
-    agree = zero_off = 0
-    for c, n in _lz4_mutants(orc, rng, 120):
-        o0 = np.zeros(n + 16, np.uint8); o1 = np.zeros(n + 16, np.uint8); o2 = np.zeros(n + 16, np.uint8)
-        d0 = ref.LZ4_decompress_safe(ptr(c), ptr(o0), ci(len(c)), ci(n))
-        d1 = orc.orc_lz4_decompress_safe(ptr(c), ptr(o1), ci(len(c)), ci(n))
-        d2 = emu.emu_lz4_decode(ptr(c), ci(len(c)), ptr(o2), ci(n))
-        assert (d0 < 0) == (d1 < 0) == (d2 < 0), (d0, d1, d2)
-        if d0 >= 0:
-            assert d0 == d1 == d2
-            assert (o0[:d0] == o1[:d0]).all() and (o0[:d0] == o2[:d0]).all()
-            agree += 1
-        assert (o2[n:] == 0).all()
-    assert agree > 10
+    t, accepted = Transcript(), 0
+    for i, (c, n) in enumerate(_lz4_mutants(orc, rng, 120)):
+        t.group(i)
+        o = np.zeros(n + 16, np.uint8)
+        d = decode(c, n, o)
+        t.add(max(d, -1))                                # a rejection is any negative value
+        if d >= 0:
+            t.add(o[:d])
+            accepted += 1
+    return t, accepted
 
 
-def test_lz4_offset_zero_decodes_to_zeros(orc, ref, emu):
+def test_lz4_decode_verdicts_match_reference(orc, emu):
+    t, accepted = _lz4_verdicts(orc, lambda c, n, o: orc.orc_lz4_decompress_safe(ptr(c), ptr(o), ci(len(c)), ci(n)))
+    check_transcript("lz4_mutant_verdicts", t)
+    assert accepted > 10
+    outs = []
+
+    def emu_decode(c, n, o):
+        d = emu.emu_lz4_decode(ptr(c), ci(len(c)), ptr(o), ci(n))
+        outs.append((o, n))
+        return d
+    check_transcript("lz4_mutant_verdicts", _lz4_verdicts(orc, emu_decode)[0])
+    assert all((o[n:] == 0).all() for o, n in outs)
+
+
+OFFSET_ZERO = bytes([0x1f, 0x41, 0x00, 0x00, 0x01]) + bytes([0x50]) + b"ABCDE"
+
+
+def test_lz4_offset_zero_decodes_to_zeros(orc, emu):
     """token 0x1f: 1 literal, match length 15+1+4 = 20, offset 0; then the mandatory last literals."""
-    s = bytes([0x1f, 0x41, 0x00, 0x00, 0x01]) + bytes([0x50]) + b"ABCDE"
-    c = np.frombuffer(s, np.uint8).copy()
+    c = np.frombuffer(OFFSET_ZERO, np.uint8).copy()
     n = 1 + 20 + 5
-    for lib, fn in ((ref, "LZ4_decompress_safe"), (orc, "orc_lz4_decompress_safe")):
-        o = np.full(n + 8, 0xEE, np.uint8)
-        assert getattr(lib, fn)(ptr(c), ptr(o), ci(len(c)), ci(n)) == n
-        assert bytes(o[:n]) == b"A" + bytes(20) + b"ABCDE"
+    want_n, want = golden()["lz4_offset_zero"]
+    assert want_n == n and bytes.fromhex(want) == b"A" + bytes(20) + b"ABCDE"       # what the reference does
+    o = np.full(n + 8, 0xEE, np.uint8)
+    assert orc.orc_lz4_decompress_safe(ptr(c), ptr(o), ci(len(c)), ci(n)) == n
+    assert bytes(o[:n]) == b"A" + bytes(20) + b"ABCDE"
     o = np.full(n + 8, 0xEE, np.uint8)
     assert emu.emu_lz4_decode(ptr(c), ci(len(c)), ptr(o), ci(n)) == n
     assert bytes(o[:n]) == b"A" + bytes(20) + b"ABCDE"
@@ -74,11 +89,12 @@ def _hostile_headers(src):
     return cases
 
 
-def test_hostile_header_cpu(orc, ref, emu):
+def test_hostile_header_cpu(orc, emu):
     src = gen("i32", 8192)
-    for c, destsize in _hostile_headers(src):
-        o0 = np.zeros(destsize, np.uint8); o1 = np.zeros(destsize, np.uint8); o2 = np.zeros(destsize, np.uint8)
-        r0 = ref.blosc_decompress_ctx(ptr(c), ptr(o0), sz(destsize), ci(1))
+    want = golden()["hostile_header_returns"]
+    assert len(want) == len(_hostile_headers(src))
+    for (c, destsize), r0 in zip(_hostile_headers(src), want):
+        o1 = np.zeros(destsize, np.uint8); o2 = np.zeros(destsize, np.uint8)
         r1 = orc.orc_decompress_ctx(ptr(c), ptr(o1), sz(destsize), ci(1))
         r2 = emu.blosc_decompress_ctx(ptr(c), ptr(o2), sz(destsize), ci(1))
         assert r0 == r1 == r2, (bytes(c[:16]).hex(), r0, r1, r2)
@@ -139,3 +155,14 @@ def test_frame_slot_validation(emu):
     bad = fr.copy()
     bad[off1 + 4:off1 + 8] = np.frombuffer(np.int32(chunk - 4).tobytes(), np.uint8)      # nbytes != the chunk's share
     assert emu.blosc_b200_frame_decompress(ptr(bad), sz(fb), ptr(out), sz(n), ci(1)) == -1
+
+
+def reference_golden(ref, orc):
+    t = _lz4_verdicts(orc, lambda c, n, o: ref.LZ4_decompress_safe(ptr(c), ptr(o), ci(len(c)), ci(n)))[0]
+    c = np.frombuffer(OFFSET_ZERO, np.uint8).copy()
+    o = np.zeros(26 + 8, np.uint8)
+    d = ref.LZ4_decompress_safe(ptr(c), ptr(o), ci(len(c)), ci(26))
+    src = gen("i32", 8192)
+    headers = [ref.blosc_decompress_ctx(ptr(h), ptr(np.zeros(ds, np.uint8)), sz(ds), ci(1)) for h, ds in _hostile_headers(src)]
+    return {"transcripts": {"lz4_mutant_verdicts": t.digests()},
+            "lz4_offset_zero": [d, bytes(o[:max(d, 0)]).hex()], "hostile_header_returns": headers}

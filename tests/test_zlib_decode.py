@@ -4,8 +4,9 @@ The algorithm lives in a third-party library of the reference (zlib 1.3.1, vendo
 internal-complibs/ and absent from this repository), so parity is pinned on (1) the reference's
 own golden chunks compat/blosc-*-zlib*.cdata, (2) streams produced and judged by the system's
 zlib (Python's `zlib` module = the same upstream library): every level / strategy / window size,
-stored, fixed and dynamic blocks, and damaged streams must get zlib's accept/reject verdict.
-CPU: the device code inside the SIMT emulator.  GPU: through the C ABI."""
+stored, fixed and dynamic blocks, and damaged streams must get zlib's accept/reject verdict, and
+(3) chunks the reference's own zlib path wrote, stored in tests/golden/reference_zlib.npz (inputs
+kept small enough to store).  CPU: the device code inside the SIMT emulator.  GPU: through the C ABI."""
 import ctypes as C
 import glob
 import os
@@ -14,7 +15,7 @@ import zlib
 import numpy as np
 import pytest
 
-from datagen import bench_words, ci, gen, ptr, sz
+from datagen import bench_words, ci, compress, decompress, gen, golden_arrays, ptr, sz
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -135,21 +136,27 @@ def test_compat_zlib_goldens_emu(emu):
     assert emu.blosc_compress_ctx(ci(5), ci(1), sz(4), sz(1000), ptr(want), ptr(out), sz(2000), b"zlib", sz(0), ci(1)) == -5   # decode only
 
 
-def test_zlib_chunks_from_the_reference_emu(emu, ref):
-    """Chunks written by the reference's own zlib path (oracle/_ref, built with its vendored
-    zlib 1.3.1): the reference's framing (splits, raw splits, leftover block) around zlib streams."""
-    if not hasattr(ref, "zlibVersion"):
-        pytest.skip("oracle/_ref was built without zlib")
-    from datagen import compress, decompress
-    for kind, n in (("bench", 300000), ("text", 100001), ("mixed", 200000), ("rand", 50000)):
-        src = gen(kind, n, 4)
-        for ts, shuf, clevel in ((4, 1, 5), (8, 2, 1), (1, 0, 9), (3, 1, 6)):
-            cb, chunk = compress(ref, "blosc_compress_ctx", clevel, shuf, ts, src, n + 16, "zlib")
-            assert cb > 0
-            r, out = decompress(emu, "blosc_decompress_ctx", chunk, n)
-            assert r == n and (out[:n] == src).all() and (out[n:] == 0).all(), (kind, ts, shuf, clevel)
-            r2, out2 = decompress(ref, "blosc_decompress_ctx", chunk, n)
-            assert r2 == n
+CHUNKS = [(kind, n, ts, shuf, clevel) for kind, n in (("bench", 6000), ("text", 3001), ("mixed", 6000), ("rand", 1000))
+          for ts, shuf, clevel in ((4, 1, 5), (8, 2, 1), (1, 0, 9), (3, 1, 6))]
+
+
+def _chunk_key(kind, n, ts, shuf, clevel):
+    return f"chunk-{kind}-{n}-{ts}-{shuf}-{clevel}"
+
+
+def _reference_chunks():
+    stored = golden_arrays("zlib")
+    assert len(stored) == len(CHUNKS)
+    return [(kind, n, ts, shuf, clevel, gen(kind, n, 4), stored[_chunk_key(kind, n, ts, shuf, clevel)])
+            for kind, n, ts, shuf, clevel in CHUNKS]
+
+
+def test_zlib_chunks_from_the_reference_emu(emu):
+    """Chunks written by the reference's own zlib path (built with its vendored zlib 1.3.1): the
+    reference's framing (splits, raw splits, leftover block) around zlib streams."""
+    for kind, n, ts, shuf, clevel, src, chunk in _reference_chunks():
+        r, out = decompress(emu, "blosc_decompress_ctx", chunk, n)
+        assert r == n and (out[:n] == src).all() and (out[n:] == 0).all(), (kind, ts, shuf, clevel)
 
 
 @pytest.mark.gpu
@@ -168,16 +175,29 @@ def test_compat_zlib_goldens_gpu(pkg, cuda):
 
 @pytest.mark.gpu
 def test_zlib_chunks_from_the_reference_gpu(pkg, ref, cuda):
-    """Chunks written by the reference's own zlib path (oracle/_ref built with its vendored zlib):
-    several typesizes / filters / levels, 2 MiB of bench.c data and text."""
-    if not hasattr(ref, "zlibVersion"):
-        pytest.skip("oracle/_ref was built without zlib")
-    from datagen import compress
-    for kind, n in (("bench", 2 << 20), ("text", 300001), ("mixed", 1 << 20)):
+    """Chunks written by the reference's own zlib path: several typesizes / filters / levels, bench.c data,
+    text, compressible runs mixed with noise, and noise.  Where oracle/_ref was built, also 2 MiB of bench.c
+    data, text and 1 MiB of mixed data, written by the reference on the spot."""
+    if ref is not None:
+        for kind, n in (("bench", 2 << 20), ("text", 300001), ("mixed", 1 << 20)):
+            src = gen(kind, n, 4)
+            for ts, shuf, clevel in ((4, 1, 5), (8, 2, 1), (1, 0, 9), (3, 1, 6)):
+                cb, chunk = compress(ref, "blosc_compress_ctx", clevel, shuf, ts, src, n + 16, "zlib")
+                assert cb > 0
+                out = np.zeros(n + 64, np.uint8)
+                assert pkg.decompress_ctx(chunk, out, n) == n
+                assert (out[:n] == src).all() and (out[n:] == 0).all(), (kind, ts, shuf, clevel)
+    for kind, n, ts, shuf, clevel, src, chunk in _reference_chunks():
+        out = np.zeros(n + 64, np.uint8)
+        assert pkg.decompress_ctx(chunk, out, n) == n
+        assert (out[:n] == src).all() and (out[n:] == 0).all()
+
+
+def reference_golden(ref, orc):
+    arrays = {}
+    for kind, n, ts, shuf, clevel in CHUNKS:
         src = gen(kind, n, 4)
-        for ts, shuf, clevel in ((4, 1, 5), (8, 2, 1), (1, 0, 9), (3, 1, 6)):
-            cb, chunk = compress(ref, "blosc_compress_ctx", clevel, shuf, ts, src, n + 16, "zlib")
-            assert cb > 0
-            out = np.zeros(n + 64, np.uint8)
-            assert pkg.decompress_ctx(chunk, out, n) == n
-            assert (out[:n] == src).all() and (out[n:] == 0).all()
+        cb, chunk = compress(ref, "blosc_compress_ctx", clevel, shuf, ts, src, n + 16, "zlib")
+        assert cb > 0 and decompress(ref, "blosc_decompress_ctx", chunk, n)[0] == n
+        arrays[_chunk_key(kind, n, ts, shuf, clevel)] = chunk[:cb].copy()
+    return arrays
