@@ -284,7 +284,7 @@ extern "C" int b2_launch_compact(const CompactArgs* a, b2_stream_t s) {
   return 0;
 }
 
-/* LZ4 streams can be decoded by a parser / copier pair of warps per stream (dev_lz4dpair.cuh).  Like the encoder's
+/* LZ4 streams can be decoded by a parser / copier pair of warps per stream (dev_lz4dec.cuh).  Like the encoder's
  * team mode it shortens the critical path of a hard stream and costs throughput where every stream is hard (a
  * descriptor per sequence on the general path): measured on the bench.c planes 0.75 -> 0.53 ms at typesize 4
  * (fast-parse chunks 0.86 -> 0.56, lz4hc 2.03 -> 1.21), but 1.04 -> 1.22 ms at typesize 2 and 0.95 -> 1.07 at typesize 8.

@@ -18,8 +18,8 @@
 #include "dev_common.cuh"
 #include "dev_inflate.cuh"
 #include "dev_lz4.cuh"
+#include "dev_lz4dec.cuh"
 #include "dev_lz4fast.cuh"
-#include "dev_lz4dpair.cuh"
 #include "dev_zstd.cuh"
 
 
@@ -71,6 +71,19 @@ DEV int ld_cg_i32(const int* p) {
 #else
   return __ldcg(p);
 #endif
+}
+
+/* End of a launch that counts finished streams: a warp that finished `mine` of them adds them to *done; true for the
+ * warp whose addition completes all nstreams (its loads after this see every other warp's writes). */
+DEV bool finished_launch(int* done, int mine, int nstreams) {
+  if (mine == 0) return false;
+  __threadfence();
+  int last = 0;
+  if (lane_id() == 0) last = atomicAdd(done, mine) + mine == nstreams;
+  last = __shfl_sync(FULLMASK, last, 0);
+  if (!last) return false;
+  __threadfence();
+  return true;
 }
 
 /* The block scan of t_blosc's ordered copy-out (blosc.c:1843-1856) by ONE warp: exclusive scan of the
@@ -151,13 +164,7 @@ __global__ void encode_kernel(EncodeArgs a) {
     __syncwarp();
   }
   /* whoever completes the stream count does the block scan and puts the counters back to zero */
-  if (mine == 0) return;
-  __threadfence();
-  int last = 0;
-  if (lane_id() == 0) last = atomicAdd(a.done, mine) + mine == a.map.nstreams;
-  last = __shfl_sync(FULLMASK, last, 0);
-  if (!last) return;
-  __threadfence();
+  if (!finished_launch(a.done, mine, a.map.nstreams)) return;
   if (a.fold_scan) warp_scan_blocks(a.scan);
   __syncwarp();
   if (lane_id() == 0) *a.done = 0;       /* (the ticket counter is never reset: warps that got no stream may still be polling it) */
@@ -207,13 +214,7 @@ __global__ void __launch_bounds__(TEAM_WARPS * 32, TEAM_CTAS_PER_SM) encode_team
   __syncwarp();
   __threadfence_block();
   bar_arrive(LZ4T_BAR_GO(0), 64); bar_arrive(LZ4T_BAR_GO(1), 64); bar_arrive(LZ4T_BAR_GO(2), 64);
-  if (mine == 0) return;
-  __threadfence();
-  int last = 0;
-  if (lane_id() == 0) last = atomicAdd(a.done, mine) + mine == a.map.nstreams;
-  last = __shfl_sync(FULLMASK, last, 0);
-  if (!last) return;
-  __threadfence();
+  if (!finished_launch(a.done, mine, a.map.nstreams)) return;
   if (a.fold_scan) warp_scan_blocks(a.scan);
   __syncwarp();
   if (lane_id() == 0) *a.done = 0;
@@ -327,13 +328,7 @@ __global__ void __launch_bounds__(FSCAN_WARPS * 32) fscan_kernel(FastArgs a) {
     mine++;
     __syncwarp();
   }
-  if (mine == 0) return;
-  __threadfence();
-  int last = 0;
-  if (lane == 0) last = atomicAdd(a.done, mine) + mine == a.map.nstreams;
-  last = __shfl_sync(FULLMASK, last, 0);
-  if (!last) return;
-  __threadfence();
+  if (!finished_launch(a.done, mine, a.map.nstreams)) return;
   if (a.fold_scan) warp_scan_blocks(a.scan);
   __syncwarp();
   if (lane == 0) *a.done = 0;
@@ -443,6 +438,23 @@ __global__ void __launch_bounds__(COMPACT_THREADS) compact_kernel(CompactArgs a)
  * word-pair form of ld_u32 would touch up to 3 bytes past cbytes */
 DEV int ld_i32(const u8* p) { return (int)((u32)p[0] | ((u32)p[1] << 8) | ((u32)p[2] << 16) | ((u32)p[3] << 24)); }
 
+/* Walk the size prefixes of a block up to one of its splits (blosc.c:760-771, :784): *so = the offset of the split's
+ * payload in the chunk, *cs = its compressed size.  Returns 0 or B2_ERR_BOUNDS. */
+DEV int locate_split(const DecodeArgs& a, int block, int split, int* so_out, int* cs_out) {
+  int so = ld_i32(a.chunk + 16 + 4ll * block);
+  int cs = 0;
+  for (int s = 0; s <= split; s++) {
+    if (so < 0 || so > a.cbytes - 4) return B2_ERR_BOUNDS;
+    cs = ld_i32(a.chunk + so);
+    so += 4;
+    if (cs < 0 || cs > a.cbytes - so) return B2_ERR_BOUNDS;
+    if (s < split) so += cs;
+  }
+  *so_out = so;
+  *cs_out = cs;
+  return 0;
+}
+
 #define DECODE_WARPS 4
 /* dynamic shared memory: DECODE_WARPS * LZ4D_SMEM bytes (per-warp ring of recent output) */
 /* One instantiation per codec: the bit-serial inflate must not cost the LZ decoders registers,
@@ -462,16 +474,8 @@ __global__ void __launch_bounds__(DECODE_WARPS * 32) decode_kernel(DecodeArgs a)
     int block, len, split;
     long long off;
     stream_locate(a.map, idx, &block, &off, &len, &split);
-    /* walk the size prefixes of this block up to our split (blosc.c:760-771, :784) */
-    int so = ld_i32(a.chunk + 16 + 4ll * block);
-    int cs = 0, err = 0;
-    for (int s = 0; s <= split; s++) {
-      if (so < 0 || so > a.cbytes - 4) { err = B2_ERR_BOUNDS; break; }
-      cs = ld_i32(a.chunk + so);
-      so += 4;
-      if (cs < 0 || cs > a.cbytes - so) { err = B2_ERR_BOUNDS; break; }
-      if (s < split) so += cs;
-    }
+    int so = 0, cs = 0;
+    int err = locate_split(a, block, split, &so, &cs);
     if (!err) {
       u8* out = a.out + (off - a.out_shift);
       const u8* src = a.chunk + so;
@@ -489,19 +493,13 @@ __global__ void __launch_bounds__(DECODE_WARPS * 32) decode_kernel(DecodeArgs a)
     mine++;
     __syncwarp();
   }
-  if (mine == 0) return;
-  __threadfence();
-  int last = 0;
-  if (lane_id() == 0) last = atomicAdd(a.done, mine) + mine == a.map.nstreams;
-  last = __shfl_sync(FULLMASK, last, 0);
-  if (!last) return;
-  __threadfence();
+  if (!finished_launch(a.done, mine, a.map.nstreams)) return;
   if (lane_id() == 0) { *a.status_out = ld_cg_i32(a.status); *a.status = 0; *a.done = 0; }
 }
 
 
 /* LZ4 chunks: one CTA of two warps per stream -- a parser that walks the tokens and a copier that owns the output
- * (dev_lz4dpair.cuh).  The parser warp alone draws tickets, checks the size prefixes, counts finished streams and
+ * (dev_lz4dec.cuh).  The parser warp alone draws tickets, checks the size prefixes, counts finished streams and
  * publishes the verdict, exactly as a warp of decode_kernel does. */
 #define PAIR_CTAS_PER_SM 12
 __global__ void __launch_bounds__(64) decode_pair_kernel(DecodeArgs a) {
@@ -510,8 +508,8 @@ __global__ void __launch_bounds__(64) decode_pair_kernel(DecodeArgs a) {
 #else
   extern __shared__ __align__(16) u8 smem[];
 #endif
-  Lz4pSlot* slots = (Lz4pSlot*)(smem + LZ4D_RING);
-  if ((threadIdx.x >> 5) == 1) { lz4_pair_copier(smem, slots); return; }
+  Lz4pSlot* slots = lz4_pair_setup(smem);
+  if (!slots) return;
   int mine = 0;
   for (;;) {
     const int idx = next_stream(a.queue, a.queue_base, a.map);
@@ -519,15 +517,8 @@ __global__ void __launch_bounds__(64) decode_pair_kernel(DecodeArgs a) {
     int block, len, split;
     long long off;
     stream_locate(a.map, idx, &block, &off, &len, &split);
-    int so = ld_i32(a.chunk + 16 + 4ll * block);
-    int cs = 0, err = 0;
-    for (int s = 0; s <= split; s++) {
-      if (so < 0 || so > a.cbytes - 4) { err = B2_ERR_BOUNDS; break; }
-      cs = ld_i32(a.chunk + so);
-      so += 4;
-      if (cs < 0 || cs > a.cbytes - so) { err = B2_ERR_BOUNDS; break; }
-      if (s < split) so += cs;
-    }
+    int so = 0, cs = 0;
+    int err = locate_split(a, block, split, &so, &cs);
     if (!err) {
       u8* out = a.out + (off - a.out_shift);
       const u8* src = a.chunk + so;
@@ -539,12 +530,6 @@ __global__ void __launch_bounds__(64) decode_pair_kernel(DecodeArgs a) {
     __syncwarp();
   }
   lz4_pair_quit(slots);
-  if (mine == 0) return;
-  __threadfence();
-  int last = 0;
-  if (lane_id() == 0) last = atomicAdd(a.done, mine) + mine == a.map.nstreams;
-  last = __shfl_sync(FULLMASK, last, 0);
-  if (!last) return;
-  __threadfence();
+  if (!finished_launch(a.done, mine, a.map.nstreams)) return;
   if (lane_id() == 0) { *a.status_out = ld_cg_i32(a.status); *a.status = 0; *a.done = 0; }
 }

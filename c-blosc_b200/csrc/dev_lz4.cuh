@@ -1,7 +1,7 @@
 /*
- * dev_lz4.cuh -- LZ4 block codec, one warp per stream, sm_100a.
+ * dev_lz4.cuh -- LZ4 block encoder, one warp per stream, sm_100a (the decoder is dev_lz4dec.cuh).
  *
- * Encoder: bit-exact replay of LZ4_compress_fast's greedy parse
+ * Bit-exact replay of LZ4_compress_fast's greedy parse
  * (reference: internal-complibs/lz4-1.10.0/lz4.c:930-1338, called from
  * blosc/blosc.c:413-420 with acceleration = 10 - clevel and maxout = neblock, i.e.
  * limitedOutput).  The sequential "probe, skip, probe" search loop (lz4.c:1043-1101)
@@ -11,16 +11,6 @@
  * the nearest lower lane with the same hash (__match_any_sync).  The first hitting
  * lane wins, and only probes up to and including it are committed to the table, so
  * the table evolves exactly as in the serial code and the output is byte-identical.
- *
- * Decoder: LZ4_decompress_safe semantics (lz4.c:2022-2445).  Four tiers: a dense path for
- * chains of literal-free sequences (one 3-byte sequence per lane, long matches with one
- * extra length byte taken inline: up to 32 sequences per step, every lane copying its own
- * match), a batch path (every lane speculatively parses the sequence that would start at
- * its input byte; the chain of real starts is resolved with one ballot or a short shuffle
- * walk and up to 11 sequences are copied 32 output bytes per instruction), a
- * single-sequence fast path, and the general path with warp-wide literal and
- * period-replicating match copies.  A per-warp shared-memory ring mirrors the last 16 KiB
- * of output so match sources do not wait behind the global stores that produced them.
  */
 #pragma once
 #include "dev_common.cuh"
@@ -708,342 +698,4 @@ DEV int lz4_encode_warp(const u8* __restrict__ s, const int n, u8* __restrict__ 
 #undef LZ4_LIMIT
 #undef LZ4_TGET
 #undef LZ4_TPUT
-}
-
-/* ---- decoder ---- */
-#ifdef SIMT_EMU
-static long long g_dbg_lz4d_batch_seqs = 0, g_dbg_lz4d_fast_seqs = 0, g_dbg_lz4d_general_seqs = 0, g_dbg_lz4d_dense_seqs = 0;
-#define LZ4D_DBG(x) do { if (lane == 0) (x)++; } while (0)
-#define LZ4D_DBGN(x, n) do { if (lane == 0) (x) += (n); } while (0)
-#else
-#define LZ4D_DBG(x) do {} while (0)
-#define LZ4D_DBGN(x, n) do {} while (0)
-#endif
-#define LZ4D_RING 16384                      /* bytes of recent output mirrored in shared memory, per warp */
-#define LZ4D_RMASK (LZ4D_RING - 1)
-#define LZ4D_BATCH_OUT 320                   /* a batch writes < 320 bytes (11 sequences x <= 27) */
-#define LZ4D_DENSE_LONG 8                    /* long matches (one extra length byte) a dense step takes inline */
-#define LZ4D_DENSE_OUT 2624                  /* a dense step writes <= 24 x 18 + 8 x 273 bytes */
-#define LZ4D_DENSE_MIN 4                     /* fewer chained 3-byte sequences than this: the 11-wide batch path is as good */
-#define LZ4D_SCRATCH 256                     /* per-warp shared scratch after the ring: sequence table + start-bit words */
-#define LZ4D_SMEM (LZ4D_RING + LZ4D_SCRATCH)
-
-/* LZ4_decompress_safe for one stream (lz4.c:2451-2456; safe-loop rules :2234-2436).
- * Returns the number of bytes written or -1.  offset==0 decodes to zeros, as in the reference.
- *
- * `ring` (LZ4D_RING bytes of warp-private shared memory) mirrors the most recent output so
- * that match sources -- a few KiB back in >99% of the sequences of shuffled data -- come
- * from shared memory instead of a global load behind the stores that produced them.
- * Fast path: token, literals (<= 8) and offset are parsed from one 12-byte register window,
- * and the whole sequence (literals + match, <= 26 bytes) is produced by one predicated
- * load/store step, one lane per output byte. */
-DEV int lz4_decode_warp(const u8* __restrict__ in, const int csize, u8* out, const int cap, u8* ring_ptr) {
-  const int iend = csize, oend = cap;
-  const int lane = lane_id();
-  const StreamBase ib = make_stream_base(in);
-  const smem_addr_t ring = smem_addr(ring_ptr);
-  int ip = 0, op = 0;
-  if (lane < 10) ((u32*)(ring_ptr + LZ4D_RING))[24 + lane] = 0;
-  __syncwarp();
-  int ring_lo = 0;                           /* positions [max(ring_lo, op-RING), op) are valid in the ring */
-  if (cap == 0) return (csize == 1 && in[0] == 0) ? 0 : -1;   /* lz4.c:2062-2066 */
-  if (csize == 0) return -1;
-  int dense_skip = 0, dense_back = 0;
-  for (;;) {
-    /* ---- dense path: a run of literal-free sequences, one per lane ----
-     * The byte-planes of shuffled data decode to long chains of 3-byte sequences (token with
-     * 0 literals and a 4..18 byte match, 16-bit offset).  If the sequence at ip is of that form the
-     * next one starts at ip+3, so lane l parses the 3 bytes at ip+3l and the leading run of lanes
-     * that all see this form are real sequences.  A prefix sum of the match lengths gives every
-     * lane its output position; sequences whose source lies entirely before the batch's first
-     * output byte are independent, and every lane copies its own match. */
-    if (dense_skip > 0) dense_skip--;
-    else if (ip + 112 <= iend && op + LZ4D_DENSE_OUT <= oend - LZ4_MFLIMIT) {
-      u32 b0, b1, b2;
-      ldp_win12(ib, ip + 3 * lane, b0, b1, b2);               /* bytes ip+3l .. ip+3l+11 (touches < ip+109) */
-      lz4d_prefetch(in, ip + 256 + 128 * lane, lane < 2 ? iend : 0);
-      /* Segments: lanes [c, e) see 3-byte sequences at byte shift s; the sequence that ends a
-       * segment is very often a longer literal-free match with one extra length byte (token 0x0F,
-       * offset, len): lane e takes it and the next segment starts one byte later (shift s+1). */
-      int kind = 0, ml = 0, off = 0, c = 0, sft = 0;
-      u32 w = b0;
-      for (;;) {
-        const u32 tok = w & 0xffu;
-        const unsigned okm = __ballot_sync(FULLMASK, lane >= c && (tok >> 4) == 0u && (tok & 15u) != 15u);
-        const unsigned stop = ~okm & ~((1u << c) - 1u);        /* first lane >= c that is not such a sequence */
-        const int e = stop ? __ffs((int)stop) - 1 : 32;
-        if (lane >= c && lane < e) { kind = 1; ml = (int)(tok & 15u) + 4; off = (int)((w >> 8) & 0xffffu); }
-        c = e;
-        if (e >= 32 || sft == LZ4D_DENSE_LONG) break;
-        const u32 tw = __shfl_sync(FULLMASK, w, e);
-        if ((tw & 0xffu) != 0x0fu || (tw >> 24) == 255u) break;
-        if (lane == e) { kind = 2; ml = 19 + (int)(tw >> 24); off = (int)((tw >> 8) & 0xffffu); }
-        c = e + 1; sft++;
-        if (c >= 32) break;
-        w = sft < 4 ? __funnelshift_r(b0, b1, 8u * (u32)sft) : (sft == 4 ? b1 : (sft < 8 ? __funnelshift_r(b1, b2, 8u * (u32)(sft - 4)) : b2));
-      }
-      int cnt = c;                                             /* lanes [0, cnt) hold one sequence each */
-      int incl = ml;
-#pragma unroll
-      for (int d = 1; d < 32; d <<= 1) {
-        const int t = __shfl_up_sync(FULLMASK, incl, d);
-        if (lane >= d) incl += t;
-      }
-      const int dst = op + incl - ml, match = dst - off;
-      /* first sequence that reads its own batch's output (or is invalid: off == 0, match < 0) ends the run;
-       * 8 bytes of slack because the word-wise copy below reads up to 7 bytes past the end of its source */
-      const unsigned bad = __ballot_sync(FULLMASK, lane < cnt && (off < incl + 8 || match < 0));
-      if (bad) cnt = __ffs((int)bad) - 1;
-      const unsigned longm = __ballot_sync(FULLMASK, lane < cnt && kind == 2);
-      if (cnt >= LZ4D_DENSE_MIN || longm) {
-        const int total = __shfl_sync(FULLMASK, incl, cnt - 1);
-        const bool from_ring = off <= LZ4D_RING - LZ4D_DENSE_OUT - 64 && match >= ring_lo;
-        {
-          /* every lane copies its own short match, 4 source bytes per step: from the ring (two aligned
-           * words + funnel shift) or, for far offsets, from the output in global memory */
-          const int mls = (lane < cnt && kind == 1) ? ml : 0;
-          const int mlmax = __ballot_sync(FULLMASK, mls > 16) ? 18 : (__ballot_sync(FULLMASK, mls > 8) ? 16 : 8);
-          u8* o = out + dst;
-#pragma unroll 1
-          for (int k = 0; k < mlmax; k += 4) {
-            if (k < mls) {
-              u32 v;
-              if (from_ring) {
-                const u32 m = (u32)(match + k);
-                v = __funnelshift_r(smem_ld_u32(ring, m & (LZ4D_RMASK & ~3u)), smem_ld_u32(ring, (m + 4u) & (LZ4D_RMASK & ~3u)), (m & 3u) * 8u);
-              } else v = ld_u32(out + match + k);       /* may read a few bytes past the source: they are not used */
-              const int nb = mls - k;
-              const u32 r = (u32)(dst + k);
-              o[k] = (u8)v; smem_st_u8(ring, r & LZ4D_RMASK, v);
-              if (nb > 1) { o[k + 1] = (u8)(v >> 8); smem_st_u8(ring, (r + 1u) & LZ4D_RMASK, v >> 8); }
-              if (nb > 2) { o[k + 2] = (u8)(v >> 16); smem_st_u8(ring, (r + 2u) & LZ4D_RMASK, v >> 16); }
-              if (nb > 3) { o[k + 3] = (u8)(v >> 24); smem_st_u8(ring, (r + 3u) & LZ4D_RMASK, v >> 24); }
-            }
-          }
-        }
-        /* the long ones, by the whole warp (their sources also lie before this step's output) */
-        for (unsigned tm = longm; tm; tm &= tm - 1u) {
-          const int t = __ffs((int)tm) - 1;
-          const int td = __shfl_sync(FULLMASK, dst, t), tmt = __shfl_sync(FULLMASK, match, t), tl = __shfl_sync(FULLMASK, ml, t);
-          const bool tring = __shfl_sync(FULLMASK, (int)from_ring, t) != 0;
-          for (int k = lane; k < tl; k += 32) {
-            const u32 v = tring ? smem_ld_u8(ring, (u32)(tmt + k) & LZ4D_RMASK) : (u32)out[tmt + k];
-            out[td + k] = (u8)v;
-            smem_st_u8(ring, (u32)(td + k) & LZ4D_RMASK, v);
-          }
-        }
-        __syncwarp();
-        ip += 3 * cnt + __popc(longm); op += total;
-        LZ4D_DBGN(g_dbg_lz4d_dense_seqs, cnt);
-        dense_back = 0;
-        continue;
-      }
-      /* a lone long match whose source overlaps its own output (small offsets): period copy by the warp */
-      {
-        const u32 tw = __shfl_sync(FULLMASK, b0, 0);
-        const int tlen = 19 + (int)(tw >> 24), toff = (int)((tw >> 8) & 0xffffu), tmatch = op - toff;
-        if ((tw & 0xffu) == 0x0fu && (tw >> 24) != 255u && toff != 0 && tmatch >= 0 && op + tlen <= oend - LZ4_MFLIMIT) {
-          const bool tring = toff <= LZ4D_RING - 512 && tmatch >= ring_lo;
-          for (int k = lane; k < tlen; k += 32) {             /* sources are all before `op`: no lane waits for another */
-            const int src = tmatch + (toff >= tlen ? k : k % toff);
-            const u32 v = tring ? smem_ld_u8(ring, (u32)src & LZ4D_RMASK) : (u32)out[src];
-            out[op + k] = (u8)v;
-            smem_st_u8(ring, (u32)(op + k) & LZ4D_RMASK, v);
-          }
-          __syncwarp();
-          ip += 4; op += tlen;
-          LZ4D_DBG(g_dbg_lz4d_dense_seqs);
-          dense_back = 0;
-          continue;
-        }
-      }
-      dense_back = dense_back < 8 ? dense_back + 1 : 8;   /* not that kind of data right here: back off */
-      dense_skip = dense_back;
-    }
-    /* ---- batch path: up to 11 short sequences per round ----
-     * Lane l speculates that a sequence starts at input byte ip+l and parses it from its own
-     * 12-byte window.  Sequences whose offset reaches back past everything this batch can write
-     * (>= LZ4D_BATCH_OUT) cannot depend on each other, so once the chain of real starts is known
-     * (one ballot when every sequence is the 3-byte literal-free form, a shuffle walk otherwise)
-     * all their output bytes are produced 32 per instruction. */
-    if (ip + 49 <= iend && op + LZ4D_BATCH_OUT <= oend - LZ4_MFLIMIT) {   /* a 9-literal sequence of lane 31 ends at ip+41 <= iend-8 (lz4.c:2289) */
-      u32 b0, b1, b2;
-      ldp_win12(ib, ip + lane, b0, b1, b2);
-      const u32 token = b0 & 0xffu;
-      const int lit = (int)(token >> 4), mln = (int)(token & 15u);
-      const int ob = 1 + lit;                                  /* window byte of the 16-bit offset (valid for lit <= 9: token, literals and offset fit the 12-byte window) */
-      const u32 ow = ob < 4 ? __funnelshift_r(b0, b1, 8u * ob) : (ob < 8 ? __funnelshift_r(b1, b2, 8u * (ob - 4)) : b2 >> (8u * ((ob - 8) & 3)));
-      const int off = (int)(ow & 0xffffu);
-      const int L = 3 + lit, O = lit + mln + 4;
-      const bool good = lit <= 9 && mln != 15 && off >= LZ4D_BATCH_OUT;
-      int nseq = 0, consumed = 0, total = 0, my_rank = -1, my_opre = 0;
-      const unsigned g3 = __ballot_sync(FULLMASK, good && lit == 0);
-      if ((g3 & 0x49249249u) == 0x49249249u) {                 /* starts at lanes 0,3,...,30 */
-        const bool real = (lane % 3) == 0;
-        const int v = real ? O : 0;
-        int incl = v;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-          const int t = __shfl_up_sync(FULLMASK, incl, d);
-          if (lane >= d) incl += t;
-        }
-        if (real) { my_rank = lane / 3; my_opre = incl - v; }
-        nseq = 11; consumed = 33;
-        total = __shfl_sync(FULLMASK, incl, 31);
-      } else {
-        const u32 packed = (good ? 1u : 0u) | ((u32)L << 1) | ((u32)O << 5);
-        int cur = 0;
-        while (cur < 32) {
-          const u32 pk = __shfl_sync(FULLMASK, packed, cur);
-          if (!(pk & 1u)) break;
-          if (lane == cur) { my_rank = nseq; my_opre = total; }
-          total += (int)((pk >> 5) & 31u);
-          cur += (int)((pk >> 1) & 15u);
-          nseq++;
-        }
-        consumed = cur;
-      }
-      if (nseq > 0) {
-        const int match = op + my_opre + lit - off;            /* meaningful on real lanes */
-        if (__ballot_sync(FULLMASK, my_rank >= 0 && match < 0)) return -1;   /* lz4.c:2356 */
-        u32* tbl = (u32*)(ring_ptr + LZ4D_RING);               /* 11 x {info, off} then 10 start-bit words */
-        u32* smask = tbl + 24;
-        if (my_rank >= 0) {
-          tbl[2 * my_rank] = (u32)my_opre | ((u32)lit << 9) | ((u32)lane << 13);
-          tbl[2 * my_rank + 1] = (u32)off;
-          atomicOr(&smask[my_opre >> 5], 1u << (my_opre & 31));
-        }
-        __syncwarp();
-        int kbase = 0;
-        for (int r = 0; r * 32 < total; r++) {
-          const u32 w = smask[r];
-          const int y = r * 32 + lane;
-          if (y < total) {
-            const int k = kbase + __popc(w & ((2u << lane) - 1u)) - 1;
-            const u32 e0 = tbl[2 * k], offk = tbl[2 * k + 1];
-            const int opre = (int)(e0 & 511u), litk = (int)((e0 >> 9) & 15u), lanek = (int)(e0 >> 13);
-            const int j = y - opre;
-            u32 v;
-            if (j < litk) v = in[ip + lanek + 1 + j];
-            else {
-              const int src = op + opre + litk - (int)offk + (j - litk);
-              const int m0 = op + opre + litk - (int)offk;
-              if ((int)offk <= LZ4D_RING - LZ4D_BATCH_OUT - 64 && m0 >= ring_lo) v = smem_ld_u8(ring, (u32)src & LZ4D_RMASK);
-              else v = out[src];
-            }
-            out[op + y] = (u8)v;
-            smem_st_u8(ring, (u32)(op + y) & LZ4D_RMASK, v);
-          }
-          kbase += __popc(w);
-        }
-        __syncwarp();
-        if (lane < 10) smask[lane] = 0;
-        __syncwarp();
-        ip += consumed; op += total;
-        LZ4D_DBGN(g_dbg_lz4d_batch_seqs, nseq);
-        continue;
-      }
-    }
-    /* ---- single-sequence fast path: short sequence, source strictly before its own output ---- */
-    if (ip + 20 <= iend) {
-      u32 b0, b1, b2;
-      ldp_win12(ib, ip, b0, b1, b2);
-      const u32 token = b0 & 0xffu;
-      const int lit = (int)(token >> 4), mln = (int)(token & 15u);
-      if (lit <= 9 && mln != 15) {
-        const int ml = mln + 4, total = lit + ml;
-        const int ob = 1 + lit;
-        const u32 ow = ob < 4 ? __funnelshift_r(b0, b1, 8u * ob) : (ob < 8 ? __funnelshift_r(b1, b2, 8u * (ob - 4)) : b2 >> (8u * (ob - 8)));
-        const int off = (int)(ow & 0xffffu);
-        const int match = op + lit - off;
-        if (off >= total && op + total <= oend - LZ4_MFLIMIT) { /* no self-overlap; far from the end of the block */
-          if (match < 0) return -1;                            /* lz4.c:2356 (off == 0 cannot get here: off >= total >= 4) */
-          const bool use_ring = off <= LZ4D_RING - 64 && match >= ring_lo;
-          if (lane < total) {
-            u32 v;
-            if (lane < lit) v = in[ip + 1 + lane];
-            else if (use_ring) v = smem_ld_u8(ring, (u32)(match + lane - lit) & LZ4D_RMASK);
-            else v = out[match + lane - lit];
-            out[op + lane] = (u8)v;
-            smem_st_u8(ring, (u32)(op + lane) & LZ4D_RMASK, v);
-          }
-          __syncwarp();
-          ip += 3 + lit; op += total;
-          LZ4D_DBG(g_dbg_lz4d_fast_seqs);
-          continue;
-        }
-      }
-    }
-    /* ---- general path ---- */
-    LZ4D_DBG(g_dbg_lz4d_general_seqs);
-    const u32 token = in[ip++];
-    int len = (int)(token >> 4);
-    if (len == 15) {                                          /* read_variable_length(ip, iend-15, 1) */
-      u32 sb;
-      if (ip >= iend - 15) return -1;
-      do {
-        sb = in[ip++];
-        len += (int)sb;
-        if (ip > iend - 15) return -1;
-        if (len > oend) return -1;                            /* same verdict as the cpy>oend test below, no int overflow */
-      } while (sb == 255);
-    }
-    int cpy = op + len;
-    const bool last = cpy > oend - LZ4_MFLIMIT || ip + len > iend - (2 + 1 + LZ4_LASTLITERALS);   /* lz4.c:2289-2331 */
-    if (last && (ip + len != iend || cpy > oend)) return -1;
-    for (int k = lane; k < len; k += 32) {                    /* literals -> output (+ ring) */
-      const u32 v = in[ip + k];
-      out[op + k] = (u8)v;
-      smem_st_u8(ring, (u32)(op + k) & LZ4D_RMASK, v);
-    }
-    if (len > LZ4D_RING - 64) ring_lo = cpy - (LZ4D_RING - 64) > ring_lo ? cpy - (LZ4D_RING - 64) : ring_lo;
-    if (last) { op += len; break; }
-    ip += len; op = cpy;
-    const int off = (int)in[ip] | ((int)in[ip + 1] << 8);
-    ip += 2;
-    const int match = op - off;
-    len = (int)(token & 15u);
-    if (len == 15) {                                          /* read_variable_length(ip, iend-4, 0) */
-      u32 sb;
-      do {
-        sb = in[ip++];
-        len += (int)sb;
-        if (ip > iend - LZ4_LASTLITERALS + 1) return -1;
-        if (len > oend) return -1;                            /* keeps `len` from overflowing on hostile input */
-      } while (sb == 255);
-    }
-    len += 4;
-    if (match < 0) return -1;                                 /* lz4.c:2356 */
-    cpy = op + len;
-    if (cpy > oend - LZ4_LASTLITERALS) return -1;             /* lz4.c:2423 */
-    __syncwarp();                                             /* earlier output must be visible to all lanes */
-    if (off == 0) {
-      /* not a valid stream, but LZ4_decompress_safe accepts it: every copy routine first clears the
-       * destination word ("silence msan warning when offset==0", lz4.c:2386-2390; LZ4_memcpy_using_offset_base)
-       * and then replicates it, so the match decodes to zeros */
-      for (int k = lane; k < len; k += 32) out[op + k] = 0;
-      ring_lo = cpy;
-    } else if (len <= 2048) {
-      /* sources lie before `op`; inside the ring they are not overwritten by this copy.  Far
-       * sources are read from global memory, but the output still goes into the ring so that it
-       * stays a mirror of the last 16 KiB */
-      const bool from_ring = off <= LZ4D_RING - 2048 - 64 && match >= ring_lo;
-      for (int k0 = 0; k0 < len; k0 += 32) {
-        const int k = k0 + lane;
-        if (k < len) {
-          const int src = match + (off >= len ? k : k % off);
-          const u32 v = from_ring ? smem_ld_u8(ring, (u32)src & LZ4D_RMASK) : (u32)out[src];
-          out[op + k] = (u8)v;
-          smem_st_u8(ring, (u32)(op + k) & LZ4D_RMASK, v);
-        }
-      }
-    } else {
-      warp_copy_match(out, op, match, len);                   /* global sources; ring no longer mirrors this span */
-      ring_lo = cpy;
-    }
-    __syncwarp();
-    op = cpy;
-  }
-  __syncwarp();
-  return op;
 }

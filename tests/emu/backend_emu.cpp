@@ -212,9 +212,8 @@ int emu_lz4_decode(const unsigned char* src, int csize, unsigned char* dst, int 
 int emu_lz4_decode_pair(const unsigned char* src, int csize, unsigned char* dst, int cap) {
   int result = 0;
   simt::launch(simt::Dim3(1), simt::Dim3(64), LZ4P_SMEM, [&] {
-    unsigned char* smem = simt::g_dynsmem;
-    Lz4pSlot* slots = (Lz4pSlot*)(smem + LZ4D_RING);
-    if ((threadIdx.x >> 5) == 1) { lz4_pair_copier(smem, slots); return; }
+    Lz4pSlot* slots = lz4_pair_setup(simt::g_dynsmem);
+    if (!slots) return;
     int r = lz4_pair_parse(src, csize, dst, cap, slots);
     lz4_pair_quit(slots);
     if ((threadIdx.x & 31) == 13) result = r;

@@ -55,7 +55,8 @@ def test_decoders_reject_garbage(emu, orc):
     b = np.zeros(20064, np.uint8)
     rb = orc.orc_blosclz_compress(ci(5), ptr(src), ci(20000), ptr(b), ci(20000), ci(1))
     for _ in range(150):
-        for buf, n, fo, fe in ((a, ra, "orc_lz4_decompress_safe", "emu_lz4_decode"), (b, rb, "orc_blosclz_decompress", "emu_blz_decode")):
+        for buf, n, fo, fe in ((a, ra, "orc_lz4_decompress_safe", "emu_lz4_decode"), (a, ra, "orc_lz4_decompress_safe", "emu_lz4_decode_pair"),
+                               (b, rb, "orc_blosclz_decompress", "emu_blz_decode")):
             c = buf[:n].copy()
             pos = rng.integers(0, n, 4)
             c[pos] = rng.integers(0, 256, 4, dtype=np.uint8)
@@ -213,12 +214,14 @@ def test_lz4_dense_path_on_corrupted_chains(emu, orc):
         for pos in rng.integers(0, ra, 1 + trial % 3):
             kind = trial % 4
             c[pos] = (0, 0xF0, 0x0F, int(rng.integers(0, 256)))[kind]
-        o1 = np.zeros(n + 8, np.uint8); o2 = np.zeros(n + 8, np.uint8)
+        o1 = np.zeros(n + 8, np.uint8)
         d1 = orc.orc_lz4_decompress_safe(ptr(c), ptr(o1), ci(ra), ci(n))
-        d2 = emu.emu_lz4_decode(ptr(c), ci(ra), ptr(o2), ci(n))
-        assert (d1 < 0) == (d2 < 0), (trial, d1, d2)
-        if d1 >= 0:
-            assert d1 == d2 and (o1[:d1] == o2[:d1]).all() and (o2[n:] == 0).all(), trial
+        for decode in (emu.emu_lz4_decode, emu.emu_lz4_decode_pair):
+            o2 = np.zeros(n + 8, np.uint8)
+            d2 = decode(ptr(c), ci(ra), ptr(o2), ci(n))
+            assert (d1 < 0) == (d2 < 0), (trial, decode.__name__, d1, d2)
+            if d1 >= 0:
+                assert d1 == d2 and (o1[:d1] == o2[:d1]).all() and (o2[n:] == 0).all(), (trial, decode.__name__)
 
 
 def test_lz4_decode_unaligned_destination(emu, orc):
@@ -261,7 +264,7 @@ def test_lz4_packed_table_is_bit_exact(emu, orc, monkeypatch):
 
 
 def test_lz4_pair_decoder_equals_single_warp_decoder(emu, orc):
-    """dev_lz4dpair.cuh (parser warp + copier warp per stream) against lz4_decode_warp and the oracle: same bytes on valid
+    """lz4_pair_parse + lz4_pair_copier (parser warp + copier warp per stream) against lz4_decode_warp and the oracle: same bytes on valid
     streams of every kind and size, same accept / reject verdict (and same bytes when accepted) on damaged ones."""
     emu.emu_lz4_decode_pair.restype = ci
     rng = np.random.default_rng(5)

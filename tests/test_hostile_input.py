@@ -72,9 +72,10 @@ def test_lz4_offset_zero_decodes_to_zeros(orc, emu):
     o = np.full(n + 8, 0xEE, np.uint8)
     assert orc.orc_lz4_decompress_safe(ptr(c), ptr(o), ci(len(c)), ci(n)) == n
     assert bytes(o[:n]) == b"A" + bytes(20) + b"ABCDE"
-    o = np.full(n + 8, 0xEE, np.uint8)
-    assert emu.emu_lz4_decode(ptr(c), ci(len(c)), ptr(o), ci(n)) == n
-    assert bytes(o[:n]) == b"A" + bytes(20) + b"ABCDE"
+    for decode in (emu.emu_lz4_decode, emu.emu_lz4_decode_pair):
+        o = np.full(n + 8, 0xEE, np.uint8)
+        assert decode(ptr(c), ci(len(c)), ptr(o), ci(n)) == n
+        assert bytes(o[:n]) == b"A" + bytes(20) + b"ABCDE"
 
 
 def _hostile_headers(src):
