@@ -20,6 +20,7 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 import datagen  # noqa: E402
 import test_abi  # noqa: E402
+import test_decoder_edges  # noqa: E402
 import test_fast_parse  # noqa: E402
 import test_hostile_input  # noqa: E402
 import test_oracle_vs_ref  # noqa: E402
@@ -46,7 +47,8 @@ def main():
 
     out = {"transcripts": {}}
     for part in (test_oracle_vs_ref.reference_golden(ref, orc), test_hostile_input.reference_golden(ref, orc),
-                 test_fast_parse.reference_golden(ref, orc), test_zstd_decode.reference_verdicts(ref, orc),
+                 test_fast_parse.reference_golden(ref, orc), test_decoder_edges.reference_golden(ref, orc),
+                 test_zstd_decode.reference_verdicts(ref, orc),
                  test_abi.reference_golden(ref_path, os.path.join(sys.argv[1], "blosc", "blosc.h"))):
         out["transcripts"].update(part.pop("transcripts", {}))
         out.update(part)
